@@ -1,7 +1,31 @@
 """TEST INFRASTRUCTURE - compact digests shared by oracle/make_golden.py (which writes them from the reference) and the tests (which
-recompute them from the oracle / the CUDA path): fixed random cotangents for the train-mode probe loss and a per-tensor gradient digest."""
+recompute them from the oracle / the CUDA path): fixed random cotangents for the train-mode probe loss, a per-tensor gradient digest and
+the row sample that keeps large outputs in a fixture under 1 MB."""
 import numpy as np
 import torch
+
+
+def keep_rows(arrs, key, step):
+    """replaces arrs[key] by every `step`-th row of it (last axis kept whole) and records the step and the full shape.  A step coprime
+    with the map sizes makes the kept rows visit every channel, anchor and upsampling phase."""
+    a = np.asarray(arrs[key])
+    arrs[f"{key}_shape"] = np.array(a.shape)
+    arrs[f"{key}_step"] = np.int64(step)
+    arrs[key] = np.ascontiguousarray(a.reshape(-1, a.shape[-1])[::step])
+
+
+def fixture_shape(g, key):
+    """the full shape of what the reference computed for `key`, also when fixture `g` keeps only rows of it"""
+    return tuple(int(v) for v in g[f"{key}_shape"]) if f"{key}_step" in g else g[key].shape
+
+
+def fixture_pair(g, key, mine):
+    """(mine, reference) over what fixture `g` stores of `key`: the whole array, or the rows keep_rows() kept (full shapes checked)"""
+    mine = np.asarray(mine)
+    if f"{key}_step" not in g:
+        return mine, g[key]
+    assert mine.shape == fixture_shape(g, key), (key, mine.shape)
+    return mine.reshape(-1, mine.shape[-1])[::int(g[f"{key}_step"])], g[key]
 
 
 def train_probe_tensors(shapes_raw, shapes_seg, seed=11):

@@ -73,6 +73,8 @@ def gen_nets(ref_yolo):
             arrs[f"raw{i}"] = r.numpy()
         for i, t in feats.items():
             arrs[f"layer{i}"] = t.numpy().astype(np.float16)  # layer taps stored as fp16 to keep fixtures small
+        if arrs["seg"].nbytes > 512 * 1024:
+            keep_rows(arrs, "seg", 3)
         np.savez_compressed(os.path.join(GOLD, f"net_{tag}.npz"), **arrs)
         print(tag, "params", sum(v.numel() for v in sd0.values()), {k: v.shape for k, v in arrs.items()},
               "z|max|", float(z.abs().max()), "seg std", float(seg.std()))
@@ -185,9 +187,10 @@ def gen_loss(ref_yolo):
     mask = torch.from_numpy(rs.randint(-1, 19, (2, 32, 64)).astype(np.int64))
     sl = ref_loss.SegmentationLosses(ignore_index=-1)(seg, mask)
     sl.backward()
-    cases.update(seg_logits=seg.detach().numpy(), seg_mask=mask.numpy(), seg_loss=sl.detach().numpy(), seg_grad=seg.grad.numpy())
     np.savez_compressed(os.path.join(GOLD, "loss_cases.npz"), **cases)
-    print("loss", {k: v.shape for k, v in cases.items() if "loss" in k or "items" in k})
+    np.savez_compressed(os.path.join(GOLD, "seg_loss_cases.npz"), seg_logits=seg.detach().numpy(), seg_mask=mask.numpy(),
+                        seg_loss=sl.detach().numpy(), seg_grad=seg.grad.numpy())      # a file of its own: each stays under 1 MB
+    print("loss", {k: v.shape for k, v in cases.items() if "loss" in k or "items" in k}, "seg", float(sl))
 
 
 def gen_letterbox():
@@ -240,16 +243,17 @@ def gen_consumers():
 
 
 # tcgen05-sized inference fixtures: every backbone / neck / head conv of these inputs runs on conv_tc_kernel (the 64x96 fixtures above
-# put every map below P2 on the CUDA-core kernel).  Stored compactly: z fp32, raw x_i fp16, low-resolution seg logits fp32, two taps.
-BIG_CASES = {
-    "s_psp_256x512": ("s_psp", "yolov5s_city_seg.yaml", 1, 256, 512, 3),
-    "m_lab_256x512": ("m_lab", "yolov5m_city_seg_lab.yaml", 1, 256, 512, 3),
-    "s_psp_512x1024": ("s_psp", "yolov5s_city_seg.yaml", 1, 512, 1024, 7),
+# put every map below P2 on the CUDA-core kernel).  Stored compactly: z fp32, raw x_i fp16, low-resolution seg logits fp32, two taps;
+# z, raw x_i and the taps keep every `step`-th row (keep_rows) so that each fixture stays under 1 MB.
+BIG_CASES = {     # name: (tag, yaml, B, H, W, input seed, row step)
+    "s_psp_256x512": ("s_psp", "yolov5s_city_seg.yaml", 1, 256, 512, 3, 3),
+    "m_lab_256x512": ("m_lab", "yolov5m_city_seg_lab.yaml", 1, 256, 512, 3, 3),
+    "s_psp_512x1024": ("s_psp", "yolov5s_city_seg.yaml", 1, 512, 1024, 7, 13),
 }
 
 
 def gen_nets_big(ref_yolo):
-    for name, (tag, yml, B, H, W, seed) in BIG_CASES.items():
+    for name, (tag, yml, B, H, W, seed, step) in BIG_CASES.items():
         cfg = synth.load_cfg(yml)
         torch.manual_seed(0)
         model = build_reference_model(ref_yolo, cfg)
@@ -273,6 +277,8 @@ def gen_nets_big(ref_yolo):
             arrs[f"raw{i}_absmax"] = np.float32(r.abs().max().item())
         for i, t in feats.items():
             arrs[f"layer{i}"] = t.numpy().astype(np.float16)
+        for k in ("z", "raw0", "raw1", "raw2", "layer9", "layer23"):
+            keep_rows(arrs, k, step)
         np.savez_compressed(os.path.join(GOLD, f"netbig_{name}.npz"), **arrs)
         print(name, {k: getattr(v, "shape", None) for k, v in arrs.items()}, os.path.getsize(os.path.join(GOLD, f"netbig_{name}.npz")) / 1e6, "MB")
 
@@ -281,7 +287,7 @@ TRAIN_CASES = {"s_psp": "yolov5s_city_seg.yaml", "s_bise": "yolov5s_city_seg_bis
                "s_base": "yolov5s_city_seg_base.yaml"}
 
 
-from oracle.digest import grad_digest, train_probe_tensors  # noqa: E402
+from oracle.digest import grad_digest, keep_rows, train_probe_tensors  # noqa: E402
 
 
 def gen_train(ref_yolo):
@@ -342,11 +348,15 @@ def gen_train(ref_yolo):
 
 def gen_ckpt(ref_yolo):
     """a checkpoint exactly as the reference's train.py:482-494 writes it (whole pickled reference `Model` in half precision inside a
-    dict), for a quarter-width yolov5s_city_seg so the fixture stays small, plus what the reference's own `attempt_load` recipe
+    dict), for a quarter-width yolov5s_city_seg whose backbone / neck stop at 128 yaml channels (32 after the width multiple; every conv
+    keeps >= 16 channels) so the fixture stays under 1 MB, plus what the reference's own `attempt_load` recipe
     (`ckpt['model'].float().fuse().eval()`, models/experimental.py:119) computes from it on a small input."""
     import copy
     cfg = synth.load_cfg("yolov5s_city_seg.yaml")
     cfg["width_multiple"] = 0.25
+    for row in cfg["backbone"] + cfg["head"]:
+        if row[2] in ("Focus", "Conv", "C3", "SPP"):
+            row[3][0] = min(row[3][0], 128)
     torch.manual_seed(7)
     model = build_reference_model(ref_yolo, cfg)
     g = torch.Generator().manual_seed(11)

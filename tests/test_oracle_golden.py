@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from oracle import restate, synth
+from oracle.digest import fixture_pair
 
 GOLD = synth.GOLDEN_DIR
 NETS = {"s_psp": "yolov5s_city_seg.yaml", "m_lab": "yolov5m_city_seg_lab.yaml", "s_bise": "yolov5s_city_seg_bise.yaml",
@@ -26,7 +27,7 @@ def test_forward_restatement_matches_reference(tag):
     out = restate.model_forward(cfg, sd, torch.from_numpy(g["x"]), keep=(0, 4, 9, 17, 23))
     # fp32 CPU both sides; differences are only BN-fold order / oneDNN kernel choice
     assert relmax(out["z"].numpy(), g["z"]) < 2e-4
-    assert relmax(out["seg"].numpy(), g["seg"]) < 2e-4
+    assert relmax(*fixture_pair(g, "seg", out["seg"].numpy())) < 2e-4
     assert relmax(out["seg_lowres"].numpy(), g["seg_lowres"]) < 2e-4
     for i in range(3):
         assert out["raw"][i].shape == g[f"raw{i}"].shape
@@ -43,7 +44,7 @@ def test_fp16_emulation_mode_is_close(tag):
     sd = synth.synth_state_dict(synth.load_manifest(tag), cfg, seed=1)
     g = np.load(os.path.join(GOLD, f"net_{tag}.npz"))
     out = restate.model_forward(cfg, sd, torch.from_numpy(g["x"]), quantised=True)
-    assert relmax(out["seg"].numpy(), g["seg"]) < 2e-2
+    assert relmax(*fixture_pair(g, "seg", out["seg"].numpy())) < 2e-2
     assert relmax(out["raw"][0].numpy(), g["raw0"]) < 2e-2
 
 
@@ -118,7 +119,7 @@ def test_det_loss_product_matches_reference(name):
 
 def test_seg_loss_matches_reference():
     from multiyolov5_b200.utils.loss import SegmentationLosses
-    g, _ = _loss_fixture()
+    g = np.load(os.path.join(GOLD, "seg_loss_cases.npz"))
     for fn in (restate.seg_ce_loss, SegmentationLosses(ignore_index=-1)):
         seg = torch.from_numpy(g["seg_logits"]).requires_grad_(True)
         loss = fn(seg, torch.from_numpy(g["seg_mask"]))
@@ -226,11 +227,11 @@ def test_forward_restatement_matches_reference_at_tensor_core_sizes(name):
     x = synth.synth_image(B, H, W, seed=int(g["seed"]))
     assert abs(float(x.double().sum()) - float(g["x_sum"])) < 1e-6 * float(g["x_sum"])
     out = restate.model_forward(cfg, sd, x, keep=(9, 23))
-    assert relmax(out["z"].numpy(), g["z"]) < 2e-4
+    assert relmax(*fixture_pair(g, "z", out["z"].numpy())) < 2e-4
     assert relmax(out["seg_lowres"].numpy(), g["seg_lowres"]) < 2e-4
     for i in range(3):
-        assert relmax(out["raw"][i].numpy(), g[f"raw{i}"].astype(np.float32)) < 1e-3      # stored as fp16
+        assert relmax(*fixture_pair(g, f"raw{i}", out["raw"][i].numpy())) < 1e-3      # stored as fp16
     for i in (9, 23):
-        assert relmax(out["layers"][i].numpy(), g[f"layer{i}"].astype(np.float32)) < 2e-3
+        assert relmax(*fixture_pair(g, f"layer{i}", out["layers"][i].numpy())) < 2e-3
     agree = float((out["seg"].argmax(1).numpy() == g["seg_argmax"]).mean())
     assert agree > 0.9999, agree
